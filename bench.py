@@ -2,7 +2,7 @@
 """bench.py — meshlet visibility pipeline on B200 (BASELINE.json metric: meshlets culled/s + tris rasterised/s,
 % of HBM roofline) with the CPU reference arm beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one frame of the hot path over the synthetic scene of BASELINE.json configs[1]
 ("1M meshlet instances, 1 camera, two-pass Hi-Z occlusion cull"): clear attachments -> cull_meshes ->
@@ -55,7 +55,32 @@ def parse_args():
     ap.add_argument("--unique-meshes", type=int, default=256,
                     help="256 = the contract scene (bounds L2-resident); 65536 makes bounds / vertex data stream from HBM")
     ap.add_argument("--parity-frames", type=int, default=3, help="N>1: frames of the pre-timing check N GPUs == 1 GPU (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last timed frame as DIR/<name>.npy (single GPU)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+# --dump-outputs: elements per array; a larger output is replaced by a fixed seeded sample of its elements, so the files stay
+# under 64 MB in all (4K images, say) and hold the same positions in every run with the same arguments
+DUMP_LIMITS = {"vis32": 3_000_000, "depth": 3_000_000, "visible_meshlet_instances": 2_000_000, "counters": 4}
+
+
+def dump_outputs(out_dir, vis32, depth, visible, counts):
+    """One frame's outputs as a caller of the path receives them (capi.Renderer.render): the R32UI vis image, the D32F depth
+    image, the survivor ids (sorted: their order is atomics order) and the counters total / early / late / triangles.
+    float64 holds every uint32 exactly."""
+    arrays = {"vis32": vis32.astype(np.float64), "depth": depth.astype(np.float32),
+              "visible_meshlet_instances": np.sort(visible).astype(np.float64),
+              "counters": np.array([counts[k] for k in ("total", "early", "late", "triangles")], dtype=np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        n = DUMP_LIMITS[name]
+        if a.size > n:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peak_hbm():
@@ -206,12 +231,16 @@ def run_reference(args):
     # bounded sample: every step is one full frame of the same scene on all host threads
     for _ in range(max(0, min(args.warmup, 1))):
         cpu_frames(scene, 1, cores)
-    n = max(1, min(args.steps, 4))
+    n = args.steps
     sec, last = cpu_frames(scene, n, cores)
     value = scene.max_meshlet_instance_count / sec
+    if args.dump_outputs:
+        v32, depth = load_oracle().resolve(last["vis64"])
+        vc = last["visibility"]
+        counts = dict(total=int(vc["total"][0]), early=int(vc["early"][0]), late=int(vc["late"][0]), triangles=last["triangles"])
+        dump_outputs(args.dump_outputs, v32, depth, last["visible"][: counts["early"] + counts["late"]], counts)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": n, "warmup": min(args.warmup, 1),
-        "steps_requested": args.steps, "steps_note": "the CPU arm is capped at 4 timed frames / 1 warm-up frame (~0.1 s per frame)",
         "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "strong" if args.total_meshlets else "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": workload_config(args, scene),
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "port",
@@ -262,6 +291,8 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     multi = world > 1
+    if multi and args.dump_outputs:
+        raise SystemExit("--dump-outputs writes the outputs of one GPU: run it with --gpus 1")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the product path has no CPU fallback")
     torch.cuda.set_device(local_rank)
@@ -357,7 +388,7 @@ def main():
     dbg("parity check done", parity)
     # ---------------- warm-up (also brings the visibility mask to steady state) ----------------
     W = max(4, args.warmup)  # >= 4 so the persistent visibility mask reaches its steady state
-    K = max(1, args.steps)
+    K = args.steps
     sampler = ClockSampler(local_rank)  # samples span warm-up + timed region + per-kernel loop (all GPU-busy)
     sampler.start()
     for i in range(W):
@@ -474,6 +505,13 @@ def main():
     cnt = pipe.counters()
     if multi:
         pipe.ctx.check_status()  # survivor-gather overflow / peer time-out are errors, not footnotes
+    if args.dump_outputs:  # before the per-kernel loop below overwrites them
+        vis32 = torch.empty((h, w), dtype=torch.int32, device=dev)
+        depth = torch.empty((h, w), dtype=torch.float32, device=dev)
+        pipe.ctx.resolve_visbuffer(pipe.vis64_bufs[(K - 1) & 1].data_ptr(), w, h, vis32.data_ptr(), depth.data_ptr())
+        dump_outputs(args.dump_outputs, vis32.cpu().numpy().view(np.uint32), depth.cpu().numpy(),
+                     pipe.ctx.visible_indices(cnt["early"] + cnt["late"]), cnt)
+        del vis32, depth
 
     dbg("timed region done", ms_per_step)
     # ---------------- per-kernel durations (same steps, eager launches, one CUDA event after every stage) ----------------
